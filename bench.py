@@ -17,6 +17,8 @@ checkpoint (no weights exist offline) and synthetic frames.
 `--impl reference` times only that CPU path (rank 0), same metric/config keys.
 `--impl hf_gpu [--liger]` times the reference's own GPU path (installed transformers, bf16, flash_attention_2, through
 oracle/hf_oracle.py) on the same clip and config: the "kernel to beat" line, printed with per-phase device time.
+`--dump-outputs DIR` writes what the last timed step of the device-resident arm returned to its caller (rank 0), as .npy
+files, so that two builds can be compared output for output on the same seeded inputs (see dump_outputs).
 """
 from __future__ import annotations
 
@@ -30,6 +32,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the tree it runs from untouched (it may be read-only)
 
 import torch  # noqa: E402
 
@@ -52,6 +55,8 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-batch", action="store_true", help="skip the multi-stream (generate_batch) sweep")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last timed step as DIR/<name>.npy (rank 0)")
     return ap.parse_args()
 
 
@@ -136,7 +141,8 @@ def build_chunks(cfg, seconds, size, seed):
 
 
 def run_stream_device(eng, chunks_dev, max_new, keep_cache=False):
-    """Device-resident inputs: one generate() per chunk, ids threaded on the device."""
+    """Device-resident inputs: one generate() per chunk, ids threaded on the device. keep_cache: the last chunk's
+    GenerateOutput (its cache not released) is returned as a fifth value."""
     cache, past_ids = None, None
     n_tok = n_frames = 0
     lat = []
@@ -153,7 +159,7 @@ def run_stream_device(eng, chunks_dev, max_new, keep_cache=False):
         lat.append((time.perf_counter() - t0) / ch["frames"])
     kv = cache.get_seq_length()
     if keep_cache:
-        return n_tok, n_frames, lat, kv, cache
+        return n_tok, n_frames, lat, kv, out
     cache.release()
     return n_tok, n_frames, lat, kv
 
@@ -211,6 +217,32 @@ def run_stream_e2e(infer, path, seconds, max_new):
     kv = state["past_key_values"].get_seq_length()
     state["past_key_values"].release()
     return n_tok, n_frames, lat, kv, h2d, d2h
+
+
+KV_SAMPLE_TOKENS = 256
+
+
+def dump_outputs(out_dir, out):
+    """What one stream's last generate() call hands its caller: `sequences` (every prompt and generated id of the whole
+    stream, as the ids are threaded through the chunks) and the KV cache. The cache is sampled: the K and V rows of
+    KV_SAMPLE_TOKENS positions drawn with a fixed seed, all layers and heads, [layers, kv_heads, tokens, 128] (7B: 29 MB
+    in all). Everything is written as float64 (ids, positions) or float32 (cache, exact for bf16)."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    cache = out.past_key_values
+    n = cache.get_seq_length()
+    g = torch.Generator().manual_seed(0)
+    pos = torch.randperm(n, generator=g)[:min(KV_SAMPLE_TOKENS, n)].sort().values
+    idx = pos.to(cache.pool.device)
+    ks, vs = zip(*(cache.gather(layer) for layer in range(cache.pool.layers)))
+    arrays = {"sequences": out.sequences.double(), "kv_positions": pos.double(),
+              "kv_keys_sample": torch.stack([k[:, idx] for k in ks]).float(),
+              "kv_values_sample": torch.stack([v[:, idx] for v in vs]).float()}
+    total = sum(a.numel() * a.element_size() for a in arrays.values())
+    assert total <= 64 << 20, f"output dump of {total} bytes exceeds 64 MB"
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------------
@@ -272,7 +304,8 @@ def time_persistent_kernel(eng, chunks_dev, max_new, iters=20):
     from livecc_b200 import _cabi
 
     t = eng.config.text_config
-    _, _, _, kv, cache = run_stream_device(eng, chunks_dev, max_new, keep_cache=True)
+    _, _, _, kv, out = run_stream_device(eng, chunks_dev, max_new, keep_cache=True)
+    cache = out.past_key_values
     with torch.inference_mode():
         cache.scalars[_cabi.SC_FINISHED] = 0
     st = [cache.stream_state()]
@@ -550,8 +583,11 @@ def main():
     for k in eng.phase_ms_total:
         eng.phase_ms_total[k] = 0
     launches0 = eng.kernel_launches()
-    for _ in range(args.steps):
-        a, b, c, kv_end = run_stream_device(eng, chunks_dev, args.max_new_tokens)
+    last_out = None
+    for i in range(args.steps):
+        keep = args.dump_outputs is not None and rank == 0 and i == args.steps - 1
+        a, b, c, kv_end, *kept = run_stream_device(eng, chunks_dev, args.max_new_tokens, keep_cache=keep)
+        last_out = kept[0] if kept else None
         tok += a
         frames += b
         lat += c
@@ -561,6 +597,9 @@ def main():
     sec = e0.elapsed_time(e1) / 1e3
     clocks = sampler.stop()
     phases = dict(eng.phase_ms_total)
+    if last_out is not None:
+        dump_outputs(args.dump_outputs, last_out)
+        last_out.past_key_values.release()
 
     # ---- end-to-end arm (public API, host frames) ----
     e2e = None

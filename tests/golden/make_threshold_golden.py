@@ -1,7 +1,7 @@
 """Generates tests/golden/threshold_golden.json by executing the reference's own ThresholdLogitsProcessor
-(REF/demo/infer.py:10-23, pure torch) on fixed score vectors. Run in the build container (needs /root/reference):
+(REF/demo/infer.py:10-23, pure torch) on fixed score vectors. Run with the path of a checkout of showlab/livecc:
 
-    python tests/golden/make_threshold_golden.py
+    python tests/golden/make_threshold_golden.py /path/to/livecc
 
 The GPU test (tests/test_ops_gpu.py::test_threshold_processor_matches_reference_golden) feeds the same scores to the
 sampling kernel and must reproduce `masked` (scores[token] == -inf) and `argmax` for every call of every case.
@@ -9,26 +9,26 @@ Cases keep softmax(scores)[token] at least 1e-3 away from the threshold, except 
 probability is exactly 2^-8 in any correct fp32 softmax (the `<=` boundary itself)."""
 import json
 import os
+import sys
 
 import torch
 
-REF = "/root/reference/demo/infer.py"
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "threshold_golden.json")
 
 
-def reference_class():
-    src = open(REF).read().splitlines()
+def reference_class(ref):
+    src = open(ref).read().splitlines()
     body = "\n".join(src[9:23])  # lines 10-23: the class definition, verbatim
     assert body.lstrip().startswith("class ThresholdLogitsProcessor(LogitsProcessor):"), body[:80]
     from transformers import LogitsProcessor
 
     ns = {"torch": torch, "LogitsProcessor": LogitsProcessor}
-    exec(compile(body, REF, "exec"), ns)
+    exec(compile(body, ref, "exec"), ns)
     return ns["ThresholdLogitsProcessor"]
 
 
 def main():
-    Proc = reference_class()
+    Proc = reference_class(os.path.join(sys.argv[1], "demo", "infer.py"))
     V = 256
     g = torch.Generator().manual_seed(7)
     cases = []

@@ -1,15 +1,14 @@
-"""Executes the UNMODIFIED reference orchestrator (REF/demo/infer.py) under the import swap INTEGRATION.md §A
-describes and diffs everything it does against livecc_b200.streaming.LiveCCDemoInfer: every generate() call
+"""Diffs livecc_b200.streaming.LiveCCDemoInfer against what the UNMODIFIED reference orchestrator (REF/demo/infer.py,
+imported under the module swap INTEGRATION.md §A describes) did on the same recording mock model: every generate() call
 (ids, cache length, pixel rows, kwargs incl. the ThresholdLogitsProcessor the canonical caller REF/demo/cli.py:16-19
-asks for), every yielded ((start, stop), text) and the `state` contract. The model is a deterministic recording mock
-(this is the host-side boundary test for SURVEY.md §8 B1-B3; the arithmetic behind generate() is covered by the
-`-m gpu` parity tests). Runs only where /root/reference exists (the build container); the GPU box has no reference."""
-import importlib
-import importlib.util
+asks for), every yielded ((start, stop), text) and the `state` contract. The reference's run is stored in
+tests/golden/orchestrator_golden.json (tests/golden/make_reference_golden.py regenerates it from a reference checkout).
+The model is a deterministic recording mock (this is the host-side boundary test for SURVEY.md §8 B1-B3; the arithmetic
+behind generate() is covered by the `-m gpu` parity tests)."""
+import hashlib
+import json
 import os
-import sys
 import types
-from unittest import mock
 
 import pytest
 import torch
@@ -17,8 +16,17 @@ import torch
 from livecc_b200.config import LiveCCConfig
 from livecc_b200.processing import StubProcessor
 
-REF_INFER = "/root/reference/demo/infer.py"
-pytestmark = pytest.mark.skipif(not os.path.exists(REF_INFER), reason="reference checkout not present on this box")
+GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+CLASS_CONSTANTS = ("fps", "initial_fps_frames", "streaming_fps_frames", "initial_time_interval",
+                   "streaming_time_interval", "frame_time_interval")
+# the recorded drop-in runs: this clip, driven for 12 s, with the cli's zero threshold and with live_cc's defaults
+DROPIN_PATH, DROPIN_SECONDS = "synthetic://330x140x112@30?seed=9", 12   # 11 s of video, non-square frames
+ZERO_THRESHOLD = dict(streaming_eos_base_threshold=0.0, streaming_eos_threshold_step=0)
+
+
+def load_golden():
+    with open(os.path.join(GOLDEN_DIR, "orchestrator_golden.json")) as f:
+        return json.load(f)
 
 
 class _Cache:
@@ -58,40 +66,6 @@ class RecordingModel:
         return types.SimpleNamespace(sequences=seq, past_key_values=cache)
 
 
-def _load_reference_class(cfg, model):
-    """REF/demo/infer.py imported verbatim with the module swap of INTEGRATION.md §A."""
-    real_tf = importlib.import_module("transformers")
-    ours = importlib.import_module("livecc_b200.livecc_utils")
-
-    class _Model:
-        @classmethod
-        def from_pretrained(cls, path, **kw):
-            model.from_pretrained_kwargs = dict(path=path, **kw)
-            return model
-
-    class _Processor:
-        @classmethod
-        def from_pretrained(cls, path, **kw):
-            return StubProcessor(cfg)
-
-    tf = types.ModuleType("transformers")
-    tf.Qwen2VLForConditionalGeneration, tf.AutoProcessor = _Model, _Processor
-    tf.LogitsProcessor, tf.logging = real_tf.LogitsProcessor, real_tf.logging
-    liger, liger_t = types.ModuleType("liger_kernel"), types.ModuleType("liger_kernel.transformers")
-    liger_t.apply_liger_kernel_to_qwen2_vl = lambda *a, **k: None
-    liger.transformers = liger_t
-    qvu = types.ModuleType("qwen_vl_utils")
-    qvu.process_vision_info = lambda *a, **k: (None, None)
-    stubs = {"transformers": tf, "liger_kernel": liger, "liger_kernel.transformers": liger_t, "qwen_vl_utils": qvu,
-             "livecc_utils": ours}
-    with mock.patch.dict(sys.modules, stubs):
-        spec = importlib.util.spec_from_file_location("ref_demo_infer", REF_INFER)
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)
-        infer = mod.LiveCCDemoInfer(model_path="synthetic-checkpoint", device="cpu")
-    return mod, infer
-
-
 def _drive(infer, path, seconds, **kw):
     """REF/demo/cli.py:13-24."""
     state = {"video_path": path}
@@ -107,59 +81,78 @@ def _drive(infer, path, seconds, **kw):
     return outs, state
 
 
-@pytest.mark.parametrize("thr", [dict(streaming_eos_base_threshold=0.0, streaming_eos_threshold_step=0), dict()])
-def test_unmodified_reference_orchestrator_equals_streaming_mirror(thr):
+def record(infer, model, path, seconds, **kw):
+    """Everything one orchestrator does on a RecordingModel, as JSON data: the constructor's derived ids, every yield,
+    every generate() call, the final state, and what a call after the end of the stream yields / asks of the model.
+    The id history of each yield is kept as a SHA-256 of its ids (every yield carries the whole history)."""
+    outs, st = _drive(infer, path, seconds, **kw)
+    outs = [(*o[:5], hashlib.sha256(json.dumps(o[5]).encode()).hexdigest(), o[6]) for o in outs]
+    n_calls = len(model.calls)
+    st["video_timestamp"] = 99
+    after = list(infer.live_cc(message="", state=st))
+    rec = dict(streaming_eos_token_id=infer.streaming_eos_token_id, system_prompt_offset=infer.system_prompt_offset,
+               outs=outs, calls=model.calls[:n_calls], video_end=bool(st.get("video_end")), message=st["message"],
+               yields_after_end=len(after), calls_after_end=len(model.calls) - n_calls)
+    return json.loads(json.dumps(rec))
+
+
+@pytest.mark.parametrize("thr", [ZERO_THRESHOLD, dict()])
+def test_unmodified_reference_orchestrator_equals_streaming_mirror(thr, monkeypatch):
+    from livecc_b200 import streaming
     from livecc_b200.streaming import LiveCCDemoInfer
 
+    gold = load_golden()
+    ref = gold["dropin_zero_threshold" if thr else "dropin_default_threshold"]
     cfg = LiveCCConfig.small()
-    path = "synthetic://330x140x112@30?seed=9"   # 11 s of video, non-square frames
-    m_ref, m_own = RecordingModel(cfg), RecordingModel(cfg)
-    mod, ref = _load_reference_class(cfg, m_ref)
-    assert m_ref.from_pretrained_kwargs["torch_dtype"] == "auto" and m_ref.from_pretrained_kwargs["device_map"] == "cpu"
-    assert callable(m_ref.prepare_inputs_for_generation)          # REF/demo/infer.py:50 assigned it on our object
-    own = LiveCCDemoInfer(model=m_own, processor=StubProcessor(cfg))
-    assert ref.streaming_eos_token_id == own.streaming_eos_token_id
-    assert ref.system_prompt_offset == own.system_prompt_offset
-    for name in ("fps", "initial_fps_frames", "streaming_fps_frames", "initial_time_interval",
-                 "streaming_time_interval", "frame_time_interval"):
-        assert getattr(mod.LiveCCDemoInfer, name) == getattr(LiveCCDemoInfer, name)
-    outs_ref, st_ref = _drive(ref, path, 12, **thr)
-    outs_own, st_own = _drive(own, path, 12, **thr)
-    assert len(outs_ref) == len(outs_own) >= 9
-    for a, b in zip(outs_ref, outs_own):
+    m_own = RecordingModel(cfg)
+    loaded = {}
+
+    def from_pretrained(path, **kw):
+        loaded.update(path=path, **kw)
+        return m_own
+
+    monkeypatch.setattr(streaming.LiveCCB200ForConditionalGeneration, "from_pretrained", staticmethod(from_pretrained))
+    own = LiveCCDemoInfer(model_path="synthetic-checkpoint", device="cpu", processor=StubProcessor(cfg))
+    for key in ("torch_dtype", "device_map"):                      # REF/demo/infer.py:43-47
+        assert loaded[key] == gold["from_pretrained_kwargs"][key], key
+    assert callable(m_own.prepare_inputs_for_generation)          # REF/demo/infer.py:50 assigns it on the model
+    for name in CLASS_CONSTANTS:
+        assert getattr(LiveCCDemoInfer, name) == gold["class_constants"][name], name
+    got = record(own, m_own, DROPIN_PATH, DROPIN_SECONDS, **thr)
+    assert got["streaming_eos_token_id"] == ref["streaming_eos_token_id"]
+    assert got["system_prompt_offset"] == ref["system_prompt_offset"]
+    assert len(got["outs"]) == len(ref["outs"]) >= 9
+    for a, b in zip(ref["outs"], got["outs"]):
         assert a == b
-    assert len(m_ref.calls) == len(m_own.calls) == len(outs_ref)
-    for a, b in zip(m_ref.calls, m_own.calls):
+    assert len(got["calls"]) == len(ref["calls"]) == len(ref["outs"])
+    for a, b in zip(ref["calls"], got["calls"]):
         pa, pb = a.pop("procs"), b.pop("procs")
         assert a == b
         if thr:
-            assert pa is not None and pb is not None and [p[1:] for p in pa] == [p[1:] for p in pb]
-            assert pa[0][0] == pb[0][0] == "ThresholdLogitsProcessor"
+            assert pa is not None and pb is not None and pa == pb
+            assert pb[0][0] == "ThresholdLogitsProcessor"
         else:
             assert pa is None and pb is None
-    assert m_ref.calls[0]["max_new_tokens"] == 16 and m_ref.calls[0]["pad_token_id"] == cfg.eos_token_id
-    assert bool(st_ref.get("video_end")) == bool(st_own.get("video_end"))
-    assert st_ref["message"] == st_own["message"]
+    assert ref["calls"][0]["max_new_tokens"] == 16 and ref["calls"][0]["pad_token_id"] == cfg.eos_token_id
+    assert got["video_end"] == ref["video_end"] and got["message"] == ref["message"]
     # nothing left to do once the stream ended: both generators are empty and make no further model calls
-    st_ref["video_timestamp"] = st_own["video_timestamp"] = 99
-    assert list(ref.live_cc(message="", state=st_ref)) == [] and list(own.live_cc(message="", state=st_own)) == []
-    assert len(m_ref.calls) == len(m_own.calls)
+    assert got["yields_after_end"] == ref["yields_after_end"] == 0
+    assert got["calls_after_end"] == ref["calls_after_end"] == 0
 
 
 def test_reference_threshold_processor_is_the_golden_source():
-    """The committed golden (tests/golden/threshold_golden.json) is what the reference class produces today."""
-    import json
-
-    sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
-    try:
-        import make_threshold_golden as mk
-    finally:
-        sys.path.pop(0)
-    Proc = mk.reference_class()
-    gold = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "threshold_golden.json")))
+    """The committed golden (tests/golden/threshold_golden.json, generated by executing the reference class) follows the
+    reference's rule, spelled out here as the test's oracle: call k masks scores[token] to -inf when
+    softmax(scores)[token] <= base + step * k, and the argmax is taken after the mask."""
+    with open(os.path.join(GOLDEN_DIR, "threshold_golden.json")) as f:
+        gold = json.load(f)
     for c in gold["cases"]:
-        proc = Proc(c["token"], c["base"], c["step"])
         scores = torch.tensor(c["scores"])
+        p = torch.softmax(scores, -1)[c["token"]]
+        assert float(p) == pytest.approx(c["prob"], rel=1e-6, abs=0), c["name"]
         for k in range(c["n_calls"]):
-            s = proc(torch.zeros((1, 1), dtype=torch.long), scores.clone()[None])[0]
-            assert bool(torch.isinf(s[c["token"]])) == c["masked"][k] and int(s.argmax()) == c["argmax"][k]
+            masked = bool(p <= c["base"] + c["step"] * k)
+            s = scores.clone()
+            if masked:
+                s[c["token"]] = -float("inf")
+            assert masked == c["masked"][k] and int(s.argmax()) == c["argmax"][k], (c["name"], k)

@@ -282,22 +282,39 @@ def test_frame_selection_matches_the_reference_scan():
         assert torch.allclose(got_ts.double(), want_ts.double()) and clip.shape[0] == len(want_idx)
 
 
-def test_cv2_reader_on_a_real_demo_video():
-    """The decord stand-in on a real 1080p clip of the reference repo (only where /root/reference is mounted):
-    pts table, smart-resized streaming size for max_pixels = 384*28*28, and a 6-frame opening clip."""
-    path = "/root/reference/demo/sources/howto_fix_laptop_mute_1080p.mp4"
-    if not os.path.exists(path):
-        pytest.skip("reference demo media not mounted on this box")
+def test_cv2_reader_on_an_encoded_video(tmp_path):
+    """The decord stand-in on a real mp4 file, written here with OpenCV's MPEG-4 encoder: 25 s at 5 fps of a moving
+    pattern at 540x960 (the aspect of the 1080p demo videos). Pts table, smart-resized streaming size for
+    max_pixels = 384*28*28, and a 6-frame opening clip whose frames are the encoded ones (each decoded frame is closest
+    to the frame written at its index, within the codec's loss)."""
+    import cv2
+
     import livecc_b200.livecc_utils as U
+
+    n, fps, h, w = 125, 5.0, 540, 960
+    yy, xx = np.mgrid[0:h, 0:w]
+
+    def frame(i):  # RGB, shifted by 8 / 4 / 6 levels per frame
+        return np.stack([(xx + 8 * i) % 256, (yy + 4 * i) % 256, ((xx + yy) // 8 + 6 * i) % 256], -1).astype(np.uint8)
+
+    path = str(tmp_path / "clip.mp4")
+    writer = cv2.VideoWriter(path, cv2.VideoWriter_fourcc(*"mp4v"), fps, (w, h))
+    assert writer.isOpened()
+    for i in range(n):
+        writer.write(cv2.cvtColor(frame(i), cv2.COLOR_RGB2BGR))
+    writer.release()
 
     reader, H, W = U.get_smart_resized_video_reader(path, 384 * 28 * 28)
     assert (H, W) == (392, 728) and H % 28 == 0 and W % 28 == 0 and H * W <= 384 * 28 * 28
     reader.get_frame_timestamp(0)
     pts = torch.from_numpy(reader._frame_pts[:, 1])
-    assert len(reader) == len(pts) > 200 and 20 < float(pts[-1]) < 60 and bool((pts[1:] > pts[:-1]).all())
+    assert len(reader) == len(pts) == n and float(pts[-1]) == pytest.approx(n / fps) and bool((pts[1:] > pts[:-1]).all())
     clip, ts, idxs = U.get_smart_resized_clip(reader, H, W, torch.arange(0.0, 3.0, 0.5), pts, 0)
     assert clip.shape == (6, 3, 392, 728) and clip.dtype == torch.uint8 and len(idxs) == 6
-    assert idxs == sorted(idxs) and float(clip.float().std()) > 5.0  # real picture content
+    assert idxs == sorted(idxs) and float(clip.float().std()) > 5.0
+    for i, got in zip(idxs, reader.get_batch(idxs).asnumpy()):
+        err = {j: float(np.abs(got.astype(np.int16) - frame(j)).mean()) for j in (i - 1, i, i + 1)}
+        assert err[i] < 4.0 and err[i] < min(err[i - 1], err[i + 1]), (i, err)
     px, grid = __import__("livecc_b200.processing", fromlist=["patchify_video"]).patchify_video(clip)
     assert grid.tolist() == [[3, 28, 52]] and px.shape == (3 * 28 * 52, 1176)
 

@@ -1,7 +1,8 @@
 """The real-processor branch (SURVEY.md §8 a4/B4): `AutoProcessor.from_pretrained(model_path, use_fast=False)`
 (REF/demo/infer.py:48-49) with the UNMODIFIED transformers Qwen2VLProcessor / tokenizer / video processor, built offline by
-tests/hf_tiny_processor.py, driven by (a) livecc_b200.streaming.LiveCCDemoInfer and (b) the unmodified reference
-orchestrator, on a recording mock model. Also pins the offline StubProcessor against it: identical pixel rows, grids and
+tests/hf_tiny_processor.py, driving livecc_b200.streaming.LiveCCDemoInfer on a recording mock model, diffed against what
+the unmodified reference orchestrator did on the same processor and mock (stored in tests/golden/orchestrator_golden.json
+by tests/golden/make_reference_golden.py). Also pins the offline StubProcessor against it: identical pixel rows, grids and
 placeholder counts."""
 import os
 import sys
@@ -66,38 +67,29 @@ def test_stub_processor_agrees_with_the_real_one(real):
         assert torch.equal(a["mm_token_type_ids"].bool(), a["input_ids"] == cfg.video_token_id)
 
 
+REAL_PATH, REAL_SECONDS = "synthetic://240x112x140@30?seed=4", 9
+
+
 def test_streaming_with_the_real_processor_equals_the_reference_orchestrator(real):
     """Both orchestrators on the real HF processor: same generate() calls, same yields (REF/demo/cli.py driving)."""
-    ref_infer = "/root/reference/demo/infer.py"
-    from test_dropin_cpu import RecordingModel, _drive
+    from test_dropin_cpu import ZERO_THRESHOLD, RecordingModel, load_golden, record
 
     from livecc_b200.streaming import LiveCCDemoInfer
 
     d, proc, cfg = real
-    path = "synthetic://240x112x140@30?seed=4"
     own_model = RecordingModel(cfg)
     own = LiveCCDemoInfer(model=own_model, processor=proc)
-    outs_own, st_own = _drive(own, path, 9, streaming_eos_base_threshold=0.0, streaming_eos_threshold_step=0)
+    got = record(own, own_model, REAL_PATH, REAL_SECONDS, **ZERO_THRESHOLD)
+    outs_own = got["outs"]
     assert len(outs_own) >= 6 and all(isinstance(o[2], str) for o in outs_own)
-    first = own_model.calls[0]
+    first = got["calls"][0]
     assert first["new"].count(cfg.video_token_id) == first["rows"] // 4 and first["procs"][0][1] == own.streaming_eos_token_id
     assert own.streaming_eos_token_id == proc.tokenizer(" ...").input_ids[-1]
-    for prev, cur in zip(own_model.calls, own_model.calls[1:]):
+    for prev, cur in zip(got["calls"], got["calls"][1:]):
         assert cur["new"][:2] == [cfg.eos_token_id, cfg.newline_token_id]      # '<|im_end|>\n' glue through the real tokenizer
-    if not os.path.exists(ref_infer):
-        pytest.skip("reference checkout not present: the differential half runs in the build container only")
-    import test_dropin_cpu as T
-
-    ref_model = RecordingModel(cfg)
-    real_stub = T.StubProcessor
-    T.StubProcessor = lambda _cfg: proc     # AutoProcessor.from_pretrained(...) inside the reference returns the real processor
-    try:
-        mod, ref = T._load_reference_class(cfg, ref_model)
-    finally:
-        T.StubProcessor = real_stub
-    outs_ref, st_ref = _drive(ref, path, 9, streaming_eos_base_threshold=0.0, streaming_eos_threshold_step=0)
-    assert outs_ref == outs_own
-    for a, b in zip(ref_model.calls, own_model.calls):
-        a, b = dict(a), dict(b)
-        pa, pb = a.pop("procs"), b.pop("procs")
-        assert a == b and [p[1:] for p in pa] == [p[1:] for p in pb]
+    ref = load_golden()["real_processor"]
+    assert got["streaming_eos_token_id"] == ref["streaming_eos_token_id"]
+    assert ref["outs"] == outs_own
+    assert len(ref["calls"]) == len(got["calls"])
+    for a, b in zip(ref["calls"], got["calls"]):
+        assert a == b

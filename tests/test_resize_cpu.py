@@ -97,23 +97,20 @@ def test_oracle_matches_torchvision_on_random_sizes():
     assert np.array_equal(resize_aa.resize_bicubic_aa_u8(clip.numpy(), (60, 1)), torchvision_resize(clip, (60, 1)).numpy())  # width only
 
 
-REF_SOURCES = "/root/reference/demo/sources"
+REFERENCE_CROPS = np.load(os.path.join(os.path.dirname(__file__), "golden", "reference_video_crops.npz"))
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_SOURCES), reason="reference checkout not present (GPU box)")
 @pytest.mark.parametrize("name", ["cvpr25_vlog.mp4", "howto_fix_laptop_mute_1080p.mp4",
                                   "warriors_vs_rockets_2025wcr1_mute_1080p.mp4"])
 def test_oracle_matches_torchvision_on_the_reference_videos(name):
-    """Real decoded frames of the three demo videos (REF/demo/sources), resized to the size the demo's reader picks
-    (get_smart_resized_video_reader, max_pixels = 384*28*28 as REF/demo/infer.py:63): oracle == the reference's
-    torchvision call, bit for bit. The GPU kernel equals the oracle bit for bit (tests/test_resize_gpu.py), which closes
-    the chain kernel == torchvision on these videos without shipping the videos to the GPU box."""
-    from livecc_b200.livecc_utils import video_process_patch as vpp
-
-    reader, H, W = vpp.get_smart_resized_video_reader(os.path.join(REF_SOURCES, name), 384 * 28 * 28)
-    n = len(reader)
-    frames = torch.from_numpy(reader.get_batch([n // 3, (2 * n) // 3]).asnumpy()).permute(0, 3, 1, 2).contiguous()
-    assert frames.shape[1] == 3 and frames.dtype == torch.uint8
+    """Real decoded frames of the three demo videos (REF/demo/sources): a 135x240 block of one 1080p frame of each, stored
+    by tests/golden/make_reference_golden.py, resized to 49x91, i.e. with the scale factors of the size the demo's reader
+    picks for the whole frame (get_smart_resized_video_reader, max_pixels = 384*28*28 as REF/demo/infer.py:63 -> 392x728):
+    oracle == the reference's torchvision call, bit for bit. The GPU kernel equals the oracle bit for bit
+    (tests/test_resize_gpu.py), which closes the chain kernel == torchvision on these videos."""
+    frames = torch.from_numpy(REFERENCE_CROPS[name])[None]
+    H, W = (int(x) for x in REFERENCE_CROPS["out_size"])
+    assert frames.shape == (1, 3, 135, 240) and frames.dtype == torch.uint8 and float(frames.float().std()) > 5.0
     ref = torchvision_resize(frames, (H, W)).numpy()
     out = resize_aa.resize_bicubic_aa_u8(frames.numpy(), (H, W))
     if torch.backends.cpu.get_cpu_capability() == GOLDEN["cpu_capability"] and torch.__version__ == GOLDEN["torch"]:
